@@ -2,7 +2,7 @@
 """bench.py -- throughput of the BPE-encode hot path (BASELINE.json metric: input GB/s and
 Mtokens/s, cl100k_base, 1 GiB synthetic English-like corpus = SURVEY.md 8(d) config 2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload config2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload config2] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one batch (the whole workload of this rank).
   value    device-resident: text + doc offsets already in HBM, tokens + offsets left in HBM.  The K steps are
@@ -25,6 +25,8 @@ A "step" = one pass of the hot path over one batch (the whole workload of this r
 N > 1 (torchrun, one rank per GPU): documents shard across ranks (weak scaling: every rank has its
 own corpus of the configured size); the only exchange is an NCCL all-gather of per-rank counts.
 Every rank is gated against the oracle before any number is reported.
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last of them left in HBM (see Bench.dump_outputs),
+so that two builds run with the same arguments -- hence the same seeded inputs -- can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,6 +41,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the source tree (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -120,6 +123,13 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons),
                 "samples": len(sm), "window": window}
+
+
+def sample_positions(n: int, k: int, seed: int = 2024) -> np.ndarray:
+    """Sorted positions of a fixed, seeded sample of at most k of range(n); all of them when n <= k."""
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    return np.unique(np.random.default_rng(seed).integers(0, n, size=k, dtype=np.int64))
 
 
 def load_reference_engine(pat, ranks, special):
@@ -265,6 +275,21 @@ class Bench:
             buf.close()
         return float(np.mean(ts)), ntok, same, self.core.last_timings()
 
+    def dump_outputs(self, out_dir, n_tok, counts):
+        """Write what the last device-resident step returned -- the tokens, the per-document token offsets and the
+        {n_tokens, n_docs} counts its last kernel wrote -- as out_dir/<name>.npy in float64 (exact for these integers).
+        Tokens and offsets are a fixed, seeded sample of positions, stored as <name>_positions.npy: under 59 MB in all
+        (the 1 GiB config2 corpus encodes to over 200 M tokens)."""
+        torch = self.torch
+        os.makedirs(out_dir, exist_ok=True)
+        arrays = {"counts": np.asarray(counts, np.float64)}
+        for name, dev, n, k in (("tokens", self.d_tok, n_tok, 3 << 20), ("token_offsets", self.d_toff, self.n_docs + 1, 1 << 19)):
+            pos = sample_positions(n, k)
+            arrays[name] = dev[torch.from_numpy(pos).to(dev.device)].cpu().numpy().astype(np.float64)
+            arrays[name + "_positions"] = pos.astype(np.float64)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+
     def close(self):
         del self.d_text, self.d_off, self.d_tok, self.d_toff, self.h_text, self.h_off, self.core, self.enc
         self.torch.cuda.empty_cache()
@@ -302,7 +327,12 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the block with the other BASELINE configs")
     ap.add_argument("--no-extras", action="store_true", help="skip api / strong-scaling / one-process multi-GPU lines")
     ap.add_argument("--decode", action="store_true", help="also time the device decode of the produced tokens (next row)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -396,7 +426,7 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.SUM)
         return int(t.item()) == 0
 
-    def measure(b: Bench, steps, warmup, sample_clocks=False):
+    def measure(b: Bench, steps, warmup, sample_clocks=False, dump_dir=None):
         """parity gate (every rank) -> value -> e2e (compared with the device result); returns a dict."""
         ok, n_tok = b.parity(cores)
         if not allok(ok):
@@ -420,6 +450,8 @@ def main():
         t1 = time.perf_counter()
         barrier()
         clocks = sampler.stop(t0, t1, t_warm) if sampler else None
+        if dump_dir and rank == 0:                              # before anything else overwrites the step's outputs
+            b.dump_outputs(dump_dir, n_tok, placements[-1][0])
         per_rank = [ms_total / steps]
         if world > 1:                                           # which rank set the pace (the MAX is what counts)
             t = torch.tensor([ms_total / steps], dtype=torch.float64, device="cuda")
@@ -444,7 +476,7 @@ def main():
                 "clocks": clocks, "counts_exchanged": [int(x) for x in placements[-1][0][:, 0]] if placements else None}
 
     b = Bench(args.workload, nbytes, rank, world, local_rank, seed_offset=7919 * rank)   # weak scaling: own corpus per rank
-    m = measure(b, args.steps, args.warmup, sample_clocks=True)
+    m = measure(b, args.steps, args.warmup, sample_clocks=True, dump_dir=args.dump_outputs)
     if not m.get("parity"):
         if rank == 0:
             print(json.dumps({"error": m.get("error", "e2e result differs from the device-resident result"), "detail": m}))
